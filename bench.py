@@ -10,20 +10,27 @@ BASELINE.json's metric has two halves, both measured by the default run and prin
               train-mode statistics (the `generate_fake` of a training iteration: SyncBN batch statistics incl. the
               cross-rank exchange, spectral-norm power iteration), no grad.  One "step" = one forward over one batch.
   train_step  configs[2]: the full G+D train iteration (hinge GAN + GAN-feature losses, Adam TTUR), batch 8 per GPU,
-              512x512 synthetic; same keys as the top level (value, ms_per_step, e2e, roofline, gpu_launches).
+              512x512 synthetic, each timed step from the same starting state; same keys as the top level (value,
+              ms_per_step, e2e, roofline, gpu_launches).
 
-  value       images/s, whole job, inputs already resident in HBM, CUDA-event timed, max over ranks.  A timed BLOCK is
-              exactly --steps steps between barrier + synchronize pairs; blocks are repeated until the leg has run for
-              >= 2 s (at most 8 blocks) and the MEDIAN block is reported (all block times are listed in `blocks_ms`).
+  value       images/s, whole job, inputs already resident in HBM, CUDA-event timed, max over ranks: one timed block of
+              exactly --steps steps between barrier + synchronize pairs, after --warmup untimed steps.
   e2e         images/s through the public API with pinned HOST buffers: H2D of the data dict and D2H of the result
               (image / loss scalars) inside the timed region
   roofline    the dominant kernel timed alone, live; roofline_worst: the kernel furthest below its roofline
   cpu_baseline / --impl reference   the reference's own CPU implementation on the host cores: the UNMODIFIED reference
               code staged under baseline/_ref (kind "reference") when present, else the CPU oracle port (kind "port")
+
+--dump-outputs DIR writes, after the timed steps, what the last timed step returned (rank 0): DIR/gen_fwd_fake_image.npy,
+DIR/train_step_generated.npy (float32) and DIR/train_step_loss_<name>.npy (float64).  Weights, inputs and Python's `random`
+are seeded, so the same arguments compute from the same inputs on every run and two builds can be compared array by array.
+Every step of the train leg starts from the same weights, buffers and optimizer state (see train_step_leg), so its outputs
+too depend only on the arguments, up to the rounding of that one step's atomic gradient sums.
 """
 import argparse
 import json
 import os
+import random
 import subprocess
 import sys
 import threading
@@ -38,8 +45,8 @@ BATCH_PER_GPU = 8
 SIZE = 512
 G_FWD_GFLOP_PER_IMG = 1114.2  # SURVEY.md §8d / BASELINE.md §3 (2*MAC, convs only)
 TRAIN_GFLOP_PER_IMG = 4775.8  # SURVEY.md §8d: G step + D step, hinge GAN + GAN-feature losses
-MIN_LEG_SECONDS = 2.0
-MAX_BLOCKS = 8
+DUMP_MAX_BYTES = 64 * 2 ** 20
+DUMP_MAX_ELEMS = 7_500_000    # per array: both 8x3x512x512 images of the default run are written whole, 60 MB together
 CPU_THREADS = 32              # fixed: PyTorch's CPU convs stop scaling (and regress) beyond ~32 threads on the B200 hosts
 
 
@@ -54,7 +61,12 @@ def parse():
                          "per-GPU work: the train step with --use_ig (frozen orientation-inpainting net, run twice per iteration)")
     ap.add_argument("--batch", type=int, default=BATCH_PER_GPU)
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the outputs of the last timed step to DIR/<name>.npy")
+    a = ap.parse_args()
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the native path")
+    return a
 
 
 def peaks():
@@ -320,9 +332,9 @@ def wgrad_kernel_roofline(batch):
 
 
 # ================================================================================================ native arm
-def timed_blocks(step, steps, world):
-    """Repeat [barrier+sync | e0 | `steps` x step | e1 | barrier+sync] until >= MIN_LEG_SECONDS have been timed; every block
-    time is the max over ranks (so all ranks agree on when to stop).  Returns the list of block times in ms."""
+def timed_block(step, steps, world):
+    """[barrier+sync | e0 | `steps` x step | e1 | barrier+sync] -> (device time of the block in ms, max over ranks; host time
+    in ms to ISSUE the block, which has no synchronisation inside)."""
     import torch.distributed as dist
 
     def barrier():
@@ -330,36 +342,45 @@ def timed_blocks(step, steps, world):
             dist.barrier()
         torch.cuda.synchronize()
 
-    blocks = []
-    timed_blocks.host_ms = []          # CPU time to ISSUE each block (no synchronisation inside a block)
-    while True:
-        barrier()
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
-        t0 = time.perf_counter()
-        for _ in range(steps):
-            step()
-        timed_blocks.host_ms.append((time.perf_counter() - t0) * 1e3)
-        e1.record()
-        barrier()
-        ms = torch.tensor([e0.elapsed_time(e1)], device="cuda")
-        if world > 1:
-            dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        blocks.append(float(ms.item()))
-        if sum(blocks) >= MIN_LEG_SECONDS * 1e3 or len(blocks) >= MAX_BLOCKS:
-            return blocks
+    barrier()
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    e0.record()
+    t0 = time.perf_counter()
+    for _ in range(steps):
+        step()
+    host_ms = (time.perf_counter() - t0) * 1e3
+    e1.record()
+    barrier()
+    ms = torch.tensor([e0.elapsed_time(e1)], device="cuda")
+    if world > 1:
+        dist.all_reduce(ms, op=dist.ReduceOp.MAX)
+    return float(ms.item()), host_ms
 
 
-def median(v):
-    s = sorted(v)
-    return s[len(s) // 2] if len(s) % 2 else 0.5 * (s[len(s) // 2 - 1] + s[len(s) // 2])
+def host_array(t, dtype):
+    """`t` as a host numpy array of `dtype`; above DUMP_MAX_ELEMS elements, a sample of its flattened values at fixed seeded
+    positions (the same on every run)."""
+    f = t.detach().to(dtype)
+    if f.numel() > DUMP_MAX_ELEMS:
+        idx = torch.randperm(f.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_MAX_ELEMS].sort().values
+        f = f.reshape(-1)[idx.to(f.device)]
+    return f.cpu().numpy()
+
+
+def write_dump(path, arrays):
+    import numpy as np
+    total = sum(v.nbytes for v in arrays.values())
+    assert total <= DUMP_MAX_BYTES, "dump of %d bytes exceeds %d" % (total, DUMP_MAX_BYTES)
+    os.makedirs(path, exist_ok=True)
+    for name, v in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), v)
 
 
 INPUT_KEYS = ("label_ref", "label_tag", "image_ref", "image_tag", "orient", "noise")
 
 
-def gen_fwd_leg(a, rank, world, local, model):
-    """-> dict of the top-level keys of the JSON line."""
+def gen_fwd_leg(a, rank, world, local, model, dump):
+    """-> dict of the top-level keys of the JSON line; with --dump-outputs, rank 0 adds the last timed step's image to `dump`."""
     import torch.distributed as dist
     from michigan_b200 import _lib, precision
     from michigan_b200.synth import synthetic_batch
@@ -376,9 +397,10 @@ def gen_fwd_leg(a, rank, world, local, model):
     with torch.no_grad():
         pre = model.preprocess_input(host)
         torch.cuda.synchronize()
+        last = {}
 
         def step():
-            return model.generate_fake(pre[0], pre[2], pre[4], pre[1], pre[3], pre[5])
+            last["fake"] = model.generate_fake(pre[0], pre[2], pre[4], pre[1], pre[3], pre[5])
 
         for _ in range(a.warmup):
             step()
@@ -387,10 +409,11 @@ def gen_fwd_leg(a, rank, world, local, model):
         if rank == 0:
             sampler.start()
         l0 = _lib.launch_count()
-        blocks = timed_blocks(step, a.steps, world)
-        launches = (_lib.launch_count() - l0) // len(blocks)
+        ms_block, _ = timed_block(step, a.steps, world)
+        launches = _lib.launch_count() - l0
         clocks = sampler.stop() if rank == 0 else None
-        ms_block = median(blocks)
+        if a.dump_outputs and rank == 0:
+            dump["gen_fwd_fake_image"] = host_array(last["fake"], torch.float32)
 
         # ---- end to end through the public API with host buffers.  Every step copies its inputs from pinned host memory
         # and reads its result back into pinned host memory; like a prefetching data loader the copies run on a second
@@ -429,7 +452,7 @@ def gen_fwd_leg(a, rank, world, local, model):
             main_stream.synchronize()
 
         e2e_run(max(2, a.warmup // 2 + 1))
-        e2e_steps = a.steps * max(1, min(MAX_BLOCKS, len(blocks)))
+        e2e_steps = a.steps
         barrier()
         t0 = time.perf_counter()
         e2e_run(e2e_steps)
@@ -451,8 +474,7 @@ def gen_fwd_leg(a, rank, world, local, model):
                    "global_batch": batch * world, "parallelism": "dp%d" % world,
                    "l2": "no explicit flush: each step streams multi-GB NHWC activations (>> 126 MB L2)",
                    "algorithmic_gflop_per_image": G_FWD_GFLOP_PER_IMG,
-                   "timing": "median of %d blocks of %d steps (>= %.0f s timed)" % (len(blocks), a.steps, MIN_LEG_SECONDS)},
-        "blocks_ms": blocks,
+                   "timing": "one block of %d steps after %d warm-up steps" % (a.steps, a.warmup)},
         "achieved_tflops_step": G_FWD_GFLOP_PER_IMG * batch / ms_step,
         "e2e": {"value": world * batch * e2e_steps / t_e2e, "unit": "images/s", "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h,
                 "steps": e2e_steps,
@@ -462,8 +484,9 @@ def gen_fwd_leg(a, rank, world, local, model):
     }
 
 
-def train_step_leg(a, rank, world, local, model, use_ig=False):
-    """BASELINE.json configs[2]: one generator update + one discriminator update per step (train.py:94-101)."""
+def train_step_leg(a, rank, world, local, model, dump, use_ig=False):
+    """BASELINE.json configs[2]: one generator update + one discriminator update per step (train.py:94-101).  With
+    --dump-outputs, rank 0 adds the last timed step's generated image and losses to `dump`."""
     import torch.distributed as dist
     from michigan_b200 import _lib
     from michigan_b200.networks.sync_batchnorm import DataParallelWithCallback, exchange_backend
@@ -482,9 +505,39 @@ def train_step_leg(a, rank, world, local, model, use_ig=False):
             dist.barrier()
         torch.cuda.synchronize()
 
+    # Every step of the timed leg starts from the same state: weights and buffers of G and D, zeroed Adam moments and step
+    # counts, and Python's `random`.  The gradient sums accumulate with float atomics, and Adam turns their last-bit
+    # differences into different updates, so a state carried from step to step would make what the n-th step computes drift
+    # from run to run.  Restoring is one device copy of the model state per step (~0.5 GB), small beside the step itself.
+    for opt in (optG, optD):        # create the Adam state now: a zero gradient leaves the weights and moments unchanged
+        for group in opt.param_groups:
+            for p in group["params"]:
+                p.grad = torch.zeros_like(p)
+        opt.step()
+        opt.zero_grad(set_to_none=True)
+
+    def by_kind(tensors):           # one fused foreach launch per (device, dtype)
+        kinds = {}
+        for t in tensors:
+            kinds.setdefault((t.device, t.dtype), []).append(t)
+        return list(kinds.values())
+
+    model_state = by_kind(t for net in (model.netG, model.netD) for t in net.state_dict().values())
+    saved_state = [[t.clone() for t in ts] for ts in model_state]
+    adam_state = by_kind(v for opt in (optG, optD) for s in opt.state.values() for v in s.values() if torch.is_tensor(v))
+    saved_random = random.getstate()
+
+    def restore():
+        for dst, src in zip(model_state, saved_state):
+            torch._foreach_copy_(dst, src)
+        for ts in adam_state:
+            torch._foreach_zero_(ts)
+        random.setstate(saved_random)
+
     def step():
-        g, d, _ = train_iteration(wrap, optG, optD, dict(dev))
-        last["losses"] = {**g, **d}
+        restore()
+        g, d, generated = train_iteration(wrap, optG, optD, dict(dev))
+        last["losses"], last["generated"] = {**g, **d}, generated
 
     for _ in range(a.warmup):
         step()
@@ -493,11 +546,14 @@ def train_step_leg(a, rank, world, local, model, use_ig=False):
     if rank == 0:
         sampler.start()
     l0 = _lib.launch_count()
-    blocks = timed_blocks(step, a.steps, world)
-    host_ms = median(timed_blocks.host_ms) / a.steps
-    launches = (_lib.launch_count() - l0) // len(blocks)
+    ms_block, host_block_ms = timed_block(step, a.steps, world)
+    host_ms = host_block_ms / a.steps
+    launches = _lib.launch_count() - l0
     clocks = sampler.stop() if rank == 0 else None
-    ms_block = median(blocks)
+    if a.dump_outputs and rank == 0:
+        dump["train_step_generated"] = host_array(last["generated"], torch.float32)
+        for k, v in last["losses"].items():
+            dump["train_step_loss_" + k] = host_array(v, torch.float64)
 
     # ---- end to end: every step's inputs come from pinned HOST tensors (copied on a second stream into one of two device
     # buffers while the previous step computes - a prefetching loader) and every step ends with its loss scalars read back to the
@@ -558,9 +614,8 @@ def train_step_leg(a, rank, world, local, model, use_ig=False):
                    "l2": "no explicit flush: multi-GB activations per step",
                    "algorithmic_gflop_per_image": TRAIN_GFLOP_PER_IMG + (2 * 151.9 if use_ig else 0.0),
                    "use_ig": bool(use_ig),
-                   "timing": "median of %d blocks of %d steps" % (len(blocks), a.steps),
+                   "timing": "one block of %d steps after %d warm-up steps" % (a.steps, a.warmup),
                    "syncbn_exchange": exchange_backend(), "grad_allreduce": "in-backward staged NCCL all-reduce (AVG) of a flat fp32 buffer"},
-        "blocks_ms": blocks,
         "achieved_tflops_step": (TRAIN_GFLOP_PER_IMG + (2 * 151.9 if use_ig else 0.0)) * batch / ms_step,
         "e2e": {"value": world * batch * e2e_steps / t_e2e, "unit": "images/s", "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": 4 * nl,
                 "steps": e2e_steps,
@@ -585,6 +640,7 @@ def run_native(a):
     from michigan_b200.synth import fill_state_dict
 
     torch.manual_seed(0)
+    random.seed(0)   # the training-mode generator draws its mask dilation with Python's `random`, as the reference does
     use_ig = a.workload == "train_step_ig"
     extra = {}
     if use_ig:
@@ -604,12 +660,15 @@ def run_native(a):
     model.train()
 
     line = None
+    dump = {}
     if a.workload in ("both", "gen_fwd"):
-        line = gen_fwd_leg(a, rank, world, local, model)
+        line = gen_fwd_leg(a, rank, world, local, model, dump)
     train = None
     if a.workload in ("both", "train_step", "train_step_ig"):
-        train = train_step_leg(a, rank, world, local, model, use_ig)
+        train = train_step_leg(a, rank, world, local, model, dump, use_ig)
     if rank == 0:
+        if a.dump_outputs:
+            write_dump(a.dump_outputs, dump)
         pk, pk_kind = peaks()
         peak_tf = float(pk["bf16_tflops"])
         if line is not None:

@@ -261,9 +261,13 @@ def main():
     for n in dnames:
         out["d0_grad/" + n] = summary(gradsD0[n], stride=53)
 
-    path = os.path.join(HERE, "golden_ngf64_128.npz")
-    np.savez_compressed(path, **out)
-    print("wrote %s (%.1f KB, %d arrays)" % (path, os.path.getsize(path) / 1024, len(out)))
+    # two files, each under 1 MB: the network outputs and losses, and the intermediate / post-step state and gradients
+    state = ("tap/", "g_post", "d_post", "g_grad/", "d_grad/", "d0_grad/")
+    for name, part in (("golden_ngf64_128.npz", {k: v for k, v in out.items() if not k.startswith(state)}),
+                       ("golden_ngf64_128_state.npz", {k: v for k, v in out.items() if k.startswith(state)})):
+        path = os.path.join(HERE, name)
+        np.savez_compressed(path, **part)
+        print("wrote %s (%.1f KB, %d arrays)" % (path, os.path.getsize(path) / 1024, len(part)))
 
 
 if __name__ == "__main__":

@@ -6,11 +6,22 @@ import numpy as np
 import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-GOLDEN = os.path.join(HERE, "golden", "golden_ngf64_128.npz")
+GOLDEN = [os.path.join(HERE, "golden", f) for f in ("golden_ngf64_128.npz", "golden_ngf64_128_state.npz")]
+
+
+class _Golden(dict):
+    """The arrays of all GOLDEN files; `files` lists their names as np.load's result does."""
+
+    @property
+    def files(self):
+        return list(self)
 
 
 def load_golden():
-    z = np.load(GOLDEN)
+    z = _Golden()
+    for path in GOLDEN:
+        with np.load(path) as f:
+            z.update({k: f[k] for k in f.files})
     cfg = json.loads(bytes(z["config"]).decode())
     return z, cfg
 

@@ -1,6 +1,6 @@
 """Host-side logic that needs no GPU: state-dict layout (= the reference's checkpoint layout),
-factory/option handling, deterministic synthesis, checkpoint I/O, and - when the reference checkout
-is present (build container only) - key-for-key equality with the reference networks and the
+factory/option handling, deterministic synthesis, checkpoint I/O, key-for-key equality with the
+reference networks (recorded under tests/golden/), and - when a reference checkout is present - the
 install() drop-in."""
 import os
 import sys
@@ -108,39 +108,41 @@ def test_checkpoint_roundtrip_layout(tmp_path):
     assert all(torch.equal(v, G2.state_dict()[k]) for k, v in G.state_dict().items())
 
 
-@needs_ref
+def _layout_golden():
+    """The reference's ngf = ndf = 32 networks as recorded by tests/golden/make_golden_layout.py."""
+    import json
+    import numpy as np
+    z = np.load(os.path.join(HERE, "golden", "golden_layout_ngf32.npz"))
+    return z, json.loads(bytes(z["layout"]).decode()), json.loads(bytes(z["config"]).decode())
+
+
 def test_layout_equals_reference_key_for_key():
-    ref_shims.patch_training()
-    opt = ref_shims.ref_options(True, ["--ngf", "32", "--ndf", "32", "--crop_size", "128", "--load_size", "128"])
-    nets = ref_shims.import_reference()
-    import io
-    import contextlib
-    with contextlib.redirect_stdout(io.StringIO()):
-        refG, refD = nets.define_G(opt), nets.define_D(opt)
+    _, layout, _ = _layout_golden()
     G = networks.SPADEBGenerator(make_opt(gpu_ids=[], ngf=32, ndf=32, crop_size=128))
     D = networks.MultiscaleDiscriminator(make_opt(gpu_ids=[], ngf=32, ndf=32, crop_size=128))
-    for mine, ref in ((G, refG), (D, refD)):
-        a, b = mine.state_dict(), ref.state_dict()
-        assert list(a.keys()) == list(b.keys())
-        assert all(a[k].shape == b[k].shape and a[k].dtype == b[k].dtype for k in a)
+    for name, mine in (("G", G), ("D", D)):
+        assert [[k, list(v.shape), str(v.dtype)] for k, v in mine.state_dict().items()] == layout[name], name
 
 
-@needs_ref
 def test_same_seed_same_initial_weights_as_reference():
-    """Construction order + init_weights mirror the reference, so a torch seed reproduces its init."""
-    ref_shims.patch_training()
-    opt = ref_shims.ref_options(True, ["--ngf", "32", "--ndf", "32", "--crop_size", "128", "--load_size", "128"])
-    nets = ref_shims.import_reference()
+    """Construction order + init_weights mirror the reference, so a torch seed reproduces its init.  The recorded
+    values are compared to 1e-6 of each tensor's largest one: the CPU's normal-distribution fill may round the last bit
+    differently on another instruction set, while any other init order or scheme changes the values outright."""
     import io
     import contextlib
-    torch.manual_seed(123)
-    with contextlib.redirect_stdout(io.StringIO()):
-        refG = nets.define_G(opt)
-    torch.manual_seed(123)
+    import numpy as np
+    z, layout, cfg = _layout_golden()
+    torch.manual_seed(cfg["init_seed"])
     with contextlib.redirect_stdout(io.StringIO()):
         G = networks.create_network(networks.SPADEBGenerator, make_opt(gpu_ids=[], ngf=32, ndf=32, crop_size=128))
-    a, b = G.state_dict(), refG.state_dict()
-    assert all(torch.equal(a[k], b[k]) for k in a)
+    a = G.state_dict()
+    assert list(a.keys()) == [k for k, _, _ in layout["G"]]
+    for k, v in a.items():
+        f = v.detach().double().reshape(-1)
+        ref = z["init/" + k]
+        assert float(np.abs(f[::max(1, f.numel() // 64)].numpy() - ref).max()) <= 1e-6 * float(np.abs(ref).max()), k
+        ref_sum = float(z["init_abs_sum/" + k][0])
+        assert abs(float(f.abs().sum()) - ref_sum) <= 1e-6 * ref_sum, k
 
 
 @needs_ref
